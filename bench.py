@@ -2,6 +2,7 @@
 """Benchmark of the DSVGP minibatch hot path (BASELINE.json metric: DSVGP train points/s, ELBO fwd+bwd).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload C3|C2|C4|C5|C1] [--impl b200|reference]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
            bench.py --gpus N --steps K --warmup W
 
@@ -27,6 +28,10 @@ One JSON line is printed by rank 0:
   cpu_baseline          (N = 1) the oracle's reference-structured step on the host cores, >= 5 timed after 2 warm-ups
 `--impl reference` times only that CPU arm (rank 0), on the same `config`; every step is a bounded sample of the workload
 (the reference's shipped minibatch of 512 points: a 16384-point step would materialise a 49152^2 K_xx on the host).
+
+`--dump-outputs DIR` (rank 0) writes what the last timed step returned to its caller, in the model dtype: DIR/loss.npy and
+DIR/grad.<parameter name>.npy for every model and likelihood parameter.  Inputs and parameters are seeded, so two builds
+run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -55,6 +60,7 @@ WORKLOADS = {  # name: variant, d, M, p, dtype, N (dataset size), default per-GP
     "C5": dict(variant="dfree", d=18, M=1024, p=2, dtype="f32", N=500000, n=16384, n_ref=512, desc="uci_dfree-shaped"),
 }
 METRIC = "DSVGP train points/s (ELBO fwd+bwd)"
+DUMP_LIMIT_BYTES = 64 << 20           # --dump-outputs: larger outputs are cut to a seeded sample of their elements
 STRONG_GLOBAL_BATCH = 131072          # SURVEY.md section 8d: the headline strong-scaling point of C3
 SWEEP_N = (512, 4096, 16384)          # SURVEY.md section 8d / BASELINE.md section 2: per-GPU minibatches of the C3 sweep
 
@@ -314,6 +320,34 @@ def dist_parity(arm, n_each=512):
     return {"ok": True, "n_global": n, "loss_rel_err": err_l, "grad_rel_err_vs_unsharded": err_g, "rank_identical_gradients": identical}
 
 
+def step_outputs(arm, loss):
+    """What a caller of the training step receives: the loss and the gradient of every model and likelihood parameter."""
+    out = {"loss": loss.detach()}
+    for owner, module in (("model", arm.model), ("likelihood", arm.lik)):
+        for name, q in module.named_parameters():
+            if q.grad is not None:
+                out[f"grad.{owner}.{name}"] = q.grad.detach()
+    return out
+
+
+def dump_outputs(path, arrays, seed=0):
+    """Writes {name: tensor} as path/<name>.npy, DUMP_LIMIT_BYTES in all.  The budget is shared out smallest array first, so
+    small outputs are always whole; an array larger than its share is replaced by its flattened elements at sorted indices
+    drawn from a generator seeded with `seed` (the same indices for the same shape, so dumps of two builds stay comparable)."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    budget = DUMP_LIMIT_BYTES - 1024 * len(arrays)                          # 1 KiB per file for the .npy header
+    order = sorted(arrays, key=lambda k: arrays[k].numel())
+    for i, name in enumerate(order):
+        t = arrays[name].cpu()
+        keep = min(t.numel(), budget // (len(order) - i) // t.element_size())
+        if keep < t.numel():
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(seed))[:keep].sort().values
+            t = t.reshape(-1)[idx]
+        budget -= t.numel() * t.element_size()
+        np.save(os.path.join(path, name + ".npy"), t.numpy())
+
+
 def main():
     _guard_stdout()
     ap = argparse.ArgumentParser()
@@ -325,7 +359,13 @@ def main():
     ap.add_argument("--n-per-gpu", type=int, default=None)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip sweep / strong scaling / other workloads (headline only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the loss and parameter gradients of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU step (--impl b200)")
     wl = dict(WORKLOADS[args.workload])
     if args.n_per_gpu:
         wl["n"] = args.n_per_gpu
@@ -372,9 +412,17 @@ def main():
     for _ in range(warmup):
         arm.step(x, V, y)
     launches0 = _lib.launch_count()
+    last = [None]
+
+    def timed_step():
+        # detached: a live loss keeps its autograd graph, and the AccumulateGrad nodes of that graph (bound to this stream)
+        # would be inherited by the side-stream warm-up of the CUDA-graph capture in the sweep below and break the capture
+        last[0] = arm.step(x, V, y).detach()
     with ClockSampler(local_rank) as clk:
-        ms_step = arm.timed(lambda: arm.step(x, V, y), args.steps)
+        ms_step = arm.timed(timed_step, args.steps)
     launches = _lib.launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, step_outputs(arm, last[0]))
 
     def e2e_step():
         xb, Vb, yb = xh.to(device, non_blocking=True), Vh.to(device, non_blocking=True), yh.to(device, non_blocking=True)
