@@ -552,8 +552,9 @@ def test_training_trajectory_agrees_across_tensor_core_paths():
     from dsvgp_b200.optim import FusedAdam
 
     def run(use_tc, use_fp16, dense_d=True):
-        old = (engine.USE_TC, engine.USE_FP16, engine.DENSE_D)
-        engine.USE_TC, engine.USE_FP16, engine.DENSE_D = use_tc, use_fp16, dense_d
+        old = (engine.USE_TC, engine.USE_FP16, engine.DENSE_D, engine.WHITEN_FP64)
+        # (3xFP16 whitening pinned: "auto" would run A = W K_zx and dK_zx = W^T dA in fp64 at this n' = 1536)
+        engine.USE_TC, engine.USE_FP16, engine.DENSE_D, engine.WHITEN_FP64 = use_tc, use_fp16, dense_d, False
         engine.ENGINE._ws.clear(), engine.ENGINE._fac.clear()
         try:
             wl = dict(bench.WORKLOADS["C3"], M=64, n=512, N=5000)
@@ -576,7 +577,7 @@ def test_training_trajectory_agrees_across_tensor_core_paths():
             assert ws.tc == use_tc and ws.tch == (use_tc and use_fp16)
             return losses, float(model.covar_module.base_kernel.lengthscale), float(vd.chol_variational_covar.abs().max())
         finally:
-            engine.USE_TC, engine.USE_FP16, engine.DENSE_D = old
+            engine.USE_TC, engine.USE_FP16, engine.DENSE_D, engine.WHITEN_FP64 = old
             engine.ENGINE._ws.clear(), engine.ENGINE._fac.clear()
 
     ref, ell_ref, _ = run(False, False)            # mma.sync 3xTF32 with fp64 master sums
