@@ -8,8 +8,16 @@
 // inverse has uniform blocks:  for a 2x2 block-lower L = [[L11,0],[L21,L22]],
 //     W = [[W11, 0], [-W22 * (L21 * W11), W22]],
 // applied bottom-up; each level is two batched GEMMs.  Diagonal nb0 x nb0 blocks are factorised AND inverted
-// inside one CTA in shared memory.  Status goes to a device int (0 ok, i+1 = first non-positive pivot), never to
+// inside one CTA in shared memory.  Status goes to a device int (0 ok, i+1 = first pivot that is not positive and finite), never to
 // the host: the caller decides when to look (no hidden synchronisation).
+//
+// Known limitation (open): the panels are solved by multiplying with explicit inverses -- L21 = A21 W11^T across blocks
+// (chol_enqueue) and A_panel D^T with D = inv(L11) on the 8x8 tiles inside a block (factor_invert_smem).  That is not
+// backward stable when the diagonal block is ill-conditioned: a tiny pivot with more rows of its block after it makes
+// the factor residual max|L L^T - A| / max|A| grow with cond(L11).  Measured on a B200, two adjacent rows at
+// cos = 1 - 1e-10 (cond 7e10) give 2e-13 .. 5e-13 against LAPACK's 6e-16, unless the pair ends its block
+// (tests/test_cholesky_gpu.py::test_adjacent_near_collinear_rows, strict xfail).  K_zz at the conditioning of trained
+// states (cond <= 1e6) stays within 1.3x of LAPACK's residual.  A stable fix solves the panels by substitution (TRSM).
 #include <algorithm>
 #include <vector>
 
@@ -215,13 +223,13 @@ potrf_inv_block(const double* __restrict__ A, int64_t lda, double* __restrict__ 
         if (ok2 && a11 > 1e-30 && a11 < 1e30 && det > 1e-30 && det < 1e30) {
           rsqrt_sqrt_f64(a11, r1, l11);
           rsqrt_sqrt_f64(det, rdet, sdet);
-        } else if (ok2) {
+        } else if (ok2 && a11 < INFINITY && det < INFINITY) {
           l11 = sqrt(a11);
           r1 = 1.0 / l11;
           sdet = sqrt(det);
           rdet = 1.0 / sdet;
-        } else {
-          if (lane == 0) atomicCAS(info, 0, row_offset + k0 + k + (ok1 ? 2 : 1));
+        } else {                                       // (+inf: l22 = inf, 1/l22 = 0 would pass as a factor with info 0)
+          if (lane == 0) atomicCAS(info, 0, row_offset + k0 + k + ((ok1 && a11 < INFINITY) ? 2 : 1));
           l11 = r1 = sdet = rdet = nan("");
         }
         const double l21 = a21 * r1;
@@ -491,13 +499,13 @@ __device__ __forceinline__ void factor_invert_smem(double* __restrict__ Ls, doub
       if (ok2 && a11 > 1e-30 && a11 < 1e30 && det > 1e-30 && det < 1e30) {
         rsqrt_sqrt_f64(a11, r1, l11);
         rsqrt_sqrt_f64(det, rdet, sdet);
-      } else if (ok2) {
+      } else if (ok2 && a11 < INFINITY && det < INFINITY) {
         l11 = sqrt(a11);
         r1 = 1.0 / l11;
         sdet = sqrt(det);
         rdet = 1.0 / sdet;
-      } else {
-        if (lane == 0) atomicCAS(info, 0, row_offset + k0 + k + (ok1 ? 2 : 1));
+      } else {                                           // (+inf: l22 = inf, 1/l22 = 0 would pass as a factor with info 0)
+        if (lane == 0) atomicCAS(info, 0, row_offset + k0 + k + ((ok1 && a11 < INFINITY) ? 2 : 1));
         l11 = r1 = sdet = rdet = nan("");
       }
       const double l21 = a21 * r1;
@@ -949,6 +957,11 @@ static int chol_enqueue(double* Awork, int64_t lda, double* L, int64_t ldl, doub
                         int nlev, int* info, cudaStream_t st) {
   if (Mp <= 0) return DSVGP_OK;
   if (!Awork || !L || !W || !info || nb0 <= 0 || nb0 > 112 || (nb0 << nlev) != Mp) return DSVGP_ERR_ARG;
+  // diag_prepare and potrf_cluster read A[k,k-1] two doubles at a time: 16-byte cp.async at Aleft + i lda + c with c even and
+  // Aleft = Awork + k nb0 lda + (k-1) nb0.  That address is 16-byte aligned for every block k and row i exactly when Awork is
+  // 16-byte aligned, lda is even and, once there is more than one block, nb0 is even (chol_plan's nb0 is a multiple of 4).
+  // Every other global access of the factorisation, the inverse and their GEMMs is 8 bytes wide or checks its own alignment.
+  if ((lda & 1) != 0 || ((uintptr_t)Awork & 15) != 0 || (nlev > 0 && (nb0 & 1) != 0)) return DSVGP_ERR_ARG;
   const int nblk = 1 << nlev;
   const int nbp = (nb0 + 7) & ~7;
   if ((nbp >> 3) * (((nbp >> 3) + 2) / 3) > 16 * POTRF_MAXBLK) return DSVGP_ERR_ARG;
@@ -1074,7 +1087,7 @@ static int chol_enqueue(double* Awork, int64_t lda, double* L, int64_t ldl, doub
       cudaStream_t gs = two_chains ? side : st;
       if (two_chains) cudaStreamWaitEvent(side, sc.ev_main[k], 0);
       double* L21 = L + (o + nb0) * ldl + o;
-      // panel  L21 = A21 * W11^T   (op(B) = W11^T is upper triangular)
+      // panel  L21 = A21 * W11^T   (op(B) = W11^T is upper triangular; explicit inverse: see the limitation at the top)
       // (W11 carries explicit zeros above its diagonal, so the triangle flag only saves flops: with the rank-K kernel on, which
       //  takes dense operands only, the panel goes through it as a dense product)
       int rc = gemm1<double>(false, true, m, nb0, nb0, 1.0, Awork + (o + nb0) * lda + o, lda, W + o * ldw + o, ldw, 0.0,

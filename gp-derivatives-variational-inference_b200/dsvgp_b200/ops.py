@@ -136,6 +136,12 @@ def set_rank_update(on):
     return call_raw("dsvgp_set_rank_update", int(on))
 
 
+def set_chol_variant(v):
+    """Diagonal-block kernel of the factorisation: 3 = 4-CTA cluster kernel (default), 2 = multi-CTA update + block kernel,
+    1 = the single-CTA round-1 kernel with the batched recursive inverse.  Returns the value in force."""
+    return call_raw("dsvgp_set_chol_variant", int(v))
+
+
 def set_chol_lookahead(on):
     """Trailing updates of the factorisation split into an urgent thin part and a bulk part on its own stream (default off)."""
     return call_raw("dsvgp_set_chol_lookahead", int(bool(on)))

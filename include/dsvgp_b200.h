@@ -103,15 +103,22 @@ int dsvgp_kdir_bwd_f32f64(const float* x1, const double* u1, const double* inv1,
  * (DirectionalGradVariationalStrategy.py:72-75) and TriangularLazyTensor.inv_matmul (:181,:183).
  * dsvgp_chol_plan: padded size Mp = nb0 << nlev for an Mq x Mq matrix.  dsvgp_pad_identity_f64 writes the identity
  * padding.  dsvgp_chol_f64: Awork (destroyed) -> L (lower), W = L^-1 (lower); *info (device int) = 0 or
- * 1 + index of the first non-positive pivot.  The panel / trailing-update GEMMs of the factorisation run on a
+ * 1 + index of the first pivot that is not a positive finite number (<= 0, NaN or +inf; a pivot pair whose determinant
+ * a11 a22 - a21^2 overflows reports its second pivot).  Only the lower triangle of Awork is read.  The factorisation loads
+ * Awork two doubles at a time from the start of every block column, so Awork must be 16-byte aligned, lda even and, when
+ * nlev > 0, nb0 even; otherwise DSVGP_ERR_ARG and nothing is enqueued.  The nb0 of dsvgp_chol_plan is a multiple of 4 and
+ * every Mp x Mp tensor the library allocates qualifies.  The panel / trailing-update GEMMs of the factorisation run on a
  * library-owned side stream (one per device) that is forked from and joined back into `s` with events: from the
  * caller's point of view everything is ordered on `s`, there is still no host synchronisation, and the call stays
  * CUDA-graph capturable.  Not re-entrant from two host threads on the same device at the same time. */
 void dsvgp_chol_plan(int Mq, int* Mp_host, int* nb0_host, int* nlev_host);
 int dsvgp_pad_identity_f64(double* A, int64_t ld, int Mq, int Mp, dsvgp_stream_t s);
 /* A/B knob of the diagonal-block chain: 1 = the round-1 kernel (DMMA prologue inside the single-CTA block kernel, scalar
- * rank-8 updates and inverse), 2 (default) = a small multi-CTA kernel forms the update of the next diagonal block and the
- * block kernel does every bulk operation as 8x8 DMMA tiles.  Returns the value in force.  Results agree to rounding. */
+ * rank-8 updates and inverse) and the batched recursive inverse after the factorisation instead of the eager one;
+ * 2 = a small multi-CTA kernel forms the update of the next diagonal block and the block kernel does every bulk operation
+ * as 8x8 DMMA tiles; 3 (default) = that update and the block kernel as one launch of a 4-CTA thread-block cluster that sums
+ * its partial updates through distributed shared memory.  A single block always takes kernel 1, and so does variant 2
+ * below four blocks.  Out-of-range values select 3.  Returns the value in force.  Results agree to rounding. */
 int dsvgp_set_chol_variant(int v);
 /* 1: the factorisation's three chains (diagonal blocks; panels + trailing updates; eager inverse) run on high-priority
  * streams owned by the library, forked from / joined to the caller's stream, so that work the caller overlaps with the
