@@ -219,6 +219,9 @@ __device__ __forceinline__ float tf32_lo_part(float x) {
 // Canonical column-side directions (every row of v2 one-hot: what train_gp / eval_gp pass, directional_vi.py:87-88,
 // :292-293) are detected on the device by normalize_dirs (no host sync): then D.w and u.w are lookups, not dot
 // products, and the per-pair work drops from (1+p1)(1+p2) to (1+p1) FMAs per coordinate.
+// p1 = p2 = 0 is the plain RBF kernel (K_zx of the SVGP baseline, K_xx of a predictive covariance without directions): one
+// output row per row point, one FMA pair per coordinate and pair, the same tiles, strips and stores with Q1 = Q2 = 1.  (Its
+// backward, kdir_bwd_v4<0, 0>, takes d <= 20 like the other cases: see bwd_v4_ok.)
 constexpr int V4_TJ = 128, V4_TIB = 64;
 
 int g_bwd_vpl = 4;             // column points per lane of kdir_bwd_v4: 4, or 2 = two CTAs per SM (benchmarking knob; measured equal:
@@ -1340,12 +1343,14 @@ static int launch_fwd_v4(const float* x1, const float* u1, int n1, const float* 
   gen<<<grid, 256, smem, st>>>(x1, u1, n1, x2, w2, cidx2, canon_flag, n2, d, hyp, use_os, (float)diag_add, K, ldk, Klo, tib,
                                stream_stores, Kh, Kl, ldkh, hscale);
   CHECK_LAUNCH();
-  if (P2 > 0 && cidx2 && canon_flag) {
-    auto can = Kh ? kdir_fwd_v4<P1, P2, 2, 1> : Klo ? kdir_fwd_v4<P1, P2, 1, 1> : kdir_fwd_v4<P1, P2, 0, 1>;
-    if (smem > 48 * 1024) cudaFuncSetAttribute(can, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    can<<<grid, 256, smem, st>>>(x1, u1, n1, x2, w2, cidx2, canon_flag, n2, d, hyp, use_os, (float)diag_add, K, ldk, Klo, tib,
-                                 stream_stores, Kh, Kl, ldkh, hscale);
-    CHECK_LAUNCH();
+  if constexpr (P2 > 0) {                   // (no canonical variant without column-side directions: not even compiled)
+    if (cidx2 && canon_flag) {
+      auto can = Kh ? kdir_fwd_v4<P1, P2, 2, 1> : Klo ? kdir_fwd_v4<P1, P2, 1, 1> : kdir_fwd_v4<P1, P2, 0, 1>;
+      if (smem > 48 * 1024) cudaFuncSetAttribute(can, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+      can<<<grid, 256, smem, st>>>(x1, u1, n1, x2, w2, cidx2, canon_flag, n2, d, hyp, use_os, (float)diag_add, K, ldk, Klo, tib,
+                                   stream_stores, Kh, Kl, ldkh, hscale);
+      CHECK_LAUNCH();
+    }
   }
   return Kh ? 2 : Klo ? 1 : DSVGP_OK;       // 1: the lo companion was written too; 2: only the half split was written
 }
@@ -1365,7 +1370,7 @@ int kdir_fwd(const T* x1, const TK* u1, int n1, int p1, const T* x2, const TK* w
   if (p1 == A && p2 == B)                                                                                      \
     return launch_fwd_v4<A, B>(x1, u1, n1, x2, w2, cidx2, canon_flag, n2, d, hyp, use_os, diag_add, K, ldk, Klo, st,          \
                                static_cast<__half*>(Kh), static_cast<__half*>(Kl), ldkh, hscale);
-      V4_CASE(1, 1) V4_CASE(2, 2) V4_CASE(3, 3) V4_CASE(1, 0) V4_CASE(2, 0) V4_CASE(3, 0)
+      V4_CASE(0, 0) V4_CASE(1, 1) V4_CASE(2, 2) V4_CASE(3, 3) V4_CASE(1, 0) V4_CASE(2, 0) V4_CASE(3, 0)
 #undef V4_CASE
     }
   }
@@ -1390,8 +1395,11 @@ int kdir_diag(int n, int p, const double* hyp, int use_os, TK* out, cudaStream_t
 }
 
 // workspace (bytes) the backward needs for an (n1,p1) x (n2,p2) call
+// (p1 = p2 = 0, the plain RBF kernel of the SVGP baseline, has the same d <= 20 limit: an exact DP = 60 instantiation for the
+//  rover shape spills 0.8 KB per thread at either VPL (-Xptxas -v: 255 / 128 registers), so d > 20 stays on the blocked kernel)
 bool bwd_v4_ok(int n1, int p1, int n2, int p2, int d) {
-  return d <= 20 && n2 >= 512 && ((p1 == 1 && p2 == 1) || (p1 == 2 && p2 == 2) || (p1 == 1 && p2 == 0) || (p1 == 2 && p2 == 0));
+  return d <= 20 && n2 >= 512 &&
+         ((p1 == 0 && p2 == 0) || (p1 == 1 && p2 == 1) || (p1 == 2 && p2 == 2) || (p1 == 1 && p2 == 0) || (p1 == 2 && p2 == 0));
 }
 
 template <typename TK>
@@ -1465,7 +1473,7 @@ int kdir_bwd(const T* x1, const TK* u1, const TK* inv1, int n1, int p1, const T*
       double* part_sc = reinterpret_cast<double*>(reinterpret_cast<unsigned char*>(ws) + part_bytes);
       // coordinates padded to a multiple of 4, except for the shapes of the shipped workloads, which get an exact instantiation
       // (d = 10: 10 instead of 12 coordinate steps in both FMA phases and one 30-value butterfly; d = 18: 18 instead of 20)
-      const int DPr = ((d == 10 && p1 == 2) || (d == 18 && p2 == 0)) ? d : (d + 3) & ~3;
+      const int DPr = ((d == 10 && (p1 == 2 || p1 == 0)) || (d == 18 && p2 == 0)) ? d : (d + 3) & ~3;
       dim3 grid(nt, nrc);
       int launched = 0;
 #define BV4V(A, B, DPV, VPLV)                                                                                  \
@@ -1481,6 +1489,7 @@ int kdir_bwd(const T* x1, const TK* u1, const TK* inv1, int n1, int p1, const T*
       BV4_ALL(1, 1) BV4_ALL(2, 2) BV4_ALL(1, 0) BV4_ALL(2, 0)
       BV4(2, 0, 20) BV4(1, 0, 20)                            // d = 17..20 without data-side directions (uci_dfree-shaped, d = 18)
       BV4(2, 2, 10) BV4(2, 0, 10) BV4(2, 0, 18) BV4(1, 0, 18)
+      BV4_ALL(0, 0) BV4(0, 0, 20) BV4(0, 0, 10) BV4(0, 0, 18)                 // value-only kernel (SVGP baseline)
 #undef BV4_ALL
 #undef BV4
 #undef BV4V

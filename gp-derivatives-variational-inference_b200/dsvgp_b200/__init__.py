@@ -9,11 +9,11 @@ from .engine import ENGINE, NanError, NotPSDError
 from .optim import FusedAdam
 from .gp import (ApproximateGP, CholeskyVariationalDistribution, ConstantMean, DFreeDirectionalGradVariationalStrategy,
                  DirectionalGradVariationalStrategy, GaussianLikelihood, GradVariationalStrategy, MultivariateNormal, NGD, NaturalVariationalDistribution,
-                 PredictiveDistribution, PredictiveLogLikelihood, RBFKernelDirectionalGrad, RBFKernelGrad, ScaleKernel,
-                 VariationalELBO)
+                 PredictiveDistribution, PredictiveLogLikelihood, RBFKernel, RBFKernelDirectionalGrad, RBFKernelGrad, ScaleKernel,
+                 VariationalELBO, VariationalStrategy)
 
 __all__ = ["ENGINE", "NanError", "NotPSDError", "ApproximateGP", "CholeskyVariationalDistribution", "ConstantMean",
            "DFreeDirectionalGradVariationalStrategy", "DirectionalGradVariationalStrategy", "FusedAdam", "GaussianLikelihood",
            "GradVariationalStrategy", "MultivariateNormal", "NGD", "NaturalVariationalDistribution", "PredictiveDistribution", "PredictiveLogLikelihood",
-           "RBFKernelDirectionalGrad", "RBFKernelGrad", "ScaleKernel", "VariationalELBO"]
+           "RBFKernel", "RBFKernelDirectionalGrad", "RBFKernelGrad", "ScaleKernel", "VariationalELBO", "VariationalStrategy"]
 __version__ = "0.1.0"

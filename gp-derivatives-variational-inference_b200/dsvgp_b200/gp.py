@@ -205,6 +205,22 @@ class RBFKernelGrad(RBFKernelDirectionalGrad):
         return x1.size(-1) + 1
 
 
+class RBFKernel(RBFKernelDirectionalGrad):
+    """gpytorch.kernels.RBFKernel as the plain SVGP baseline uses it (traditional_vi.py): isotropic, key `raw_lengthscale`
+    (1, 1) under softplus.  forward(x1, x2) is the plain (n1, n2) RBF matrix -- the directional kernel with p = 0 on both
+    sides, on the same assembly kernels; diag=True (x1 == x2) is a vector of ones."""
+
+    def num_outputs_per_input(self, x1, x2):
+        return 1
+
+    def forward(self, x1, x2, diag=False, **params):
+        if diag:
+            if not (x1.shape == x2.shape and torch.equal(x1, x2)):
+                raise RuntimeError("diag=True only works when x1 == x2")
+            return torch.ones(x1.shape[-2], dtype=x1.dtype, device=x1.device)
+        return _KDir.apply(x1, x2, None, None, self.raw_lengthscale, 0, 0)
+
+
 class ScaleKernel(Module):
     """gpytorch.kernels.ScaleKernel: keys `raw_outputscale` (0-dim) and `base_kernel.*`."""
 
@@ -890,3 +906,22 @@ class GradVariationalStrategy(_DirectionalStrategyBase):
 
     def _data_directions(self, x, kwargs):
         return self._canonical(x.shape[0], x)
+
+
+class VariationalStrategy(_DirectionalStrategyBase):
+    """gpytorch.variational.VariationalStrategy as the plain SVGP baseline uses it (traditional_vi.py): whitened, over the
+    M function values at the inducing points, labels are function values only.  This is the directional strategy with p = 0
+    on both sides, on the same fused step; the gpytorch 1.4 constants are the same as there (K_zz jitter 1e-3, predictive
+    jitter 1e-4, the 1e-6 / 1e-5 / 1e-4 Cholesky ladder, the 1e-6 / 1e-10 variance floor)."""
+
+    def _p(self):
+        return 0
+
+    def _directions(self):
+        return None
+
+    def _data_directions(self, x, kwargs):
+        if kwargs.get("derivative_directions") is not None:
+            raise TypeError("VariationalStrategy models function values only: it takes no derivative_directions "
+                            "(use DirectionalGradVariationalStrategy for derivative information)")
+        return None
