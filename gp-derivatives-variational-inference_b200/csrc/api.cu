@@ -77,6 +77,20 @@ KBWD(dsvgp_kdir_bwd_f32, float, float)
 KBWD(dsvgp_kdir_bwd_f64, double, double)
 KBWD(dsvgp_kdir_bwd_f32f64, float, double)
 
+size_t dsvgp_kdir_bwd_cols_workspace_f32(int n1, int p1, int n2, int p2, int d) { return kdir_bwd_cols_workspace<float>(n1, p1, n2, p2, d); }
+size_t dsvgp_kdir_bwd_cols_workspace_f64(int n1, int p1, int n2, int p2, int d) { return kdir_bwd_cols_workspace<double>(n1, p1, n2, p2, d); }
+
+#define KBWDC(NAME, T)                                                                                             \
+  int NAME(const T* x1, const T* u1, int n1, int p1, const T* x2, const T* w2, const T* inv2, int n2, int p2, int d, \
+           const double* hyp, int use_os, const T* dK, int64_t lddk, double scale, double* gx, double* gv, void* ws, \
+           size_t ws_bytes, dsvgp_stream_t s) {                                                                    \
+    if (!x1 || !x2 || !hyp || !dK || !ws || (p1 > 0 && !u1) || (p2 > 0 && (!w2 || (gv && !inv2)))) return DSVGP_ERR_ARG; \
+    return kdir_bwd_cols<T, T>(x1, u1, n1, p1, x2, w2, inv2, n2, p2, d, hyp, use_os, dK, lddk, scale, gx, gv, ws,    \
+                               ws_bytes, ST(s));                                                                   \
+  }
+KBWDC(dsvgp_kdir_bwd_cols_f32, float)
+KBWDC(dsvgp_kdir_bwd_cols_f64, double)
+
 void dsvgp_chol_plan(int Mq, int* Mp, int* nb0, int* nlev) { chol_plan(Mq, Mp, nb0, nlev); }
 int dsvgp_pad_identity_f64(double* A, int64_t ld, int Mq, int Mp, dsvgp_stream_t s) { return pad_identity(A, ld, Mq, Mp, ST(s)); }
 int dsvgp_chol_f64(double* Awork, int64_t lda, double* L, int64_t ldl, double* W, int64_t ldw, int Mp, int nb0, int nlev, int* info, dsvgp_stream_t s) {

@@ -1138,6 +1138,186 @@ kdir_bwd_v4(const float* __restrict__ x1, const float* __restrict__ u1, int n1, 
   }
 }
 
+// ------------------------------------------------------------------------- backward, data side (fp32, vectorised)
+// d/dx2_j and d/dw_jb of sum(dK * K(x1, x2)) -- the gradient w.r.t. the data points and data-side directions of K_zx.  With
+// D = x1_i - x2_j and the coefficients e0, ea, eb, hab of kdir_bwd_v4 (which give d/dx1_i = sum_j e0 D + eb w_jb + ea u_ia):
+//   d/dx2_j  = -sum_i (e0 D + sum_b eb w_jb + sum_a ea u_ia)        (x2 enters through -D only)
+//   d/dw_jb  =  sum_i (eb D + sum_a hab u_ia)
+// One thread per column (data) point, COLS_TJ consecutive points per CTA; the CTA sweeps a chunk of row (inducing) points,
+// staged COLS_RT at a time in shared memory and read as broadcasts.  Each thread reads its own Q2 consecutive floats of every
+// upstream row (a warp: 32 * Q2 * 4 contiguous bytes), so dK is read once and coalesced and K is recomputed.  The thread's
+// column operands and its (1 + P2) * DP sums stay in registers; one fp64 partial per (row chunk, column point) goes to the
+// workspace and kdir_bwd_reduce_rows adds the chunks in a fixed order (deterministic, no atomics) and applies the
+// normalisation chain of w.  A separate kernel rather than a second output of kdir_bwd_v4, which already needs ~250 registers.
+constexpr int COLS_TJ = 256, COLS_RT = 32, COLS_CTAS = 148 * 4;
+
+// row chunks of the data-side kernel: about COLS_CTAS CTAs in all, at least 8 row points per chunk
+__host__ __device__ inline int cols_num_chunks(int n1, int n2) {
+  const int nct = (n2 + COLS_TJ - 1) / COLS_TJ, maxch = (n1 + 7) / 8;
+  int want = (COLS_CTAS + nct - 1) / nct;
+  if (want > maxch) want = maxch;
+  if (want < 1) want = 1;
+  const int pts = (n1 + want - 1) / want;
+  return (n1 + pts - 1) / pts;
+}
+
+template <int P1, int P2, int DP>
+__global__ void __launch_bounds__(COLS_TJ, 1)
+kdir_bwd_cols_v4(const float* __restrict__ x1, const float* __restrict__ u1, int n1, const float* __restrict__ x2,
+                 const float* __restrict__ w2, int n2, int d, const double* __restrict__ hyp, int use_os,
+                 const float* __restrict__ dK, int64_t lddk, int chunk_pts, double* __restrict__ part) {
+  constexpr int Q1 = P1 + 1, Q2 = P2 + 1, PA = P1 > 0 ? P1 : 1, PB = P2 > 0 ? P2 : 1;
+  __shared__ __align__(16) float rs[COLS_RT * Q1 * DP];   // [row point][Q1][DP]: x1_i then u_i1..u_iP1
+  const int tid = threadIdx.x, j = blockIdx.x * COLS_TJ + tid;
+  const bool act = j < n2;
+  const int ibeg = blockIdx.y * chunk_pts, iend = min(n1, ibeg + chunk_pts);
+
+  float xj[DP], wj[PB][DP], sx[DP], sw[PB][DP];
+#pragma unroll
+  for (int c = 0; c < DP; ++c) {
+    xj[c] = (act && c < d) ? x2[(int64_t)j * d + c] : 0.f;
+    sx[c] = 0.f;
+#pragma unroll
+    for (int b = 0; b < P2; ++b) {
+      wj[b][c] = (act && c < d) ? w2[((int64_t)j * P2 + b) * d + c] : 0.f;
+      sw[b][c] = 0.f;
+    }
+  }
+  const float ell = (float)hyp[0], os = use_os ? (float)hyp[1] : 1.f;
+  const float il2 = 1.f / (ell * ell);
+  const float* gcol = dK + (act ? (int64_t)j * Q2 : 0);
+  auto load_g = [&](int gi, float (&g)[Q1][Q2]) {
+#pragma unroll
+    for (int a = 0; a < Q1; ++a)
+#pragma unroll
+      for (int b = 0; b < Q2; ++b) g[a][b] = act ? gcol[(int64_t)(gi * Q1 + a) * lddk + b] : 0.f;
+  };
+
+  for (int i0 = ibeg; i0 < iend; i0 += COLS_RT) {
+    const int nr = min(COLS_RT, iend - i0);
+    __syncthreads();
+    for (int e = tid; e < COLS_RT * Q1 * DP; e += COLS_TJ) {
+      const int cc = e % DP, ia = e / DP, i = ia / Q1, a = ia % Q1;
+      const bool ok = i < nr && cc < d;
+      rs[e] = !ok ? 0.f : (a == 0) ? x1[(int64_t)(i0 + i) * d + cc] : u1[((int64_t)(i0 + i) * P1 + a - 1) * d + cc];
+    }
+    __syncthreads();
+    float g[Q1][Q2], gn[Q1][Q2];
+    load_g(i0, g);
+    for (int il = 0; il < nr; ++il) {
+      load_g(min(i0 + il + 1, iend - 1), gn);             // the next row point's upstream block, in flight during this one
+      const float* rb = rs + il * Q1 * DP;
+      // ---- recompute r2 = |D|^2, alpha = D.u, beta = D.w, gamma = u.w
+      float r2 = 0.f, al[PA], be[PB], ga[PA][PB];
+#pragma unroll
+      for (int a = 0; a < P1; ++a) al[a] = 0.f;
+#pragma unroll
+      for (int b = 0; b < P2; ++b) be[b] = 0.f;
+#pragma unroll
+      for (int a = 0; a < P1; ++a)
+#pragma unroll
+        for (int b = 0; b < P2; ++b) ga[a][b] = 0.f;
+#pragma unroll
+      for (int c4 = 0; c4 < DP; c4 += 4) {
+        const float4 xr = *reinterpret_cast<const float4*>(rb + c4);
+        float4 ur[PA];
+#pragma unroll
+        for (int a = 0; a < P1; ++a) ur[a] = *reinterpret_cast<const float4*>(rb + (1 + a) * DP + c4);
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+          const int c = c4 + k;
+          const float dl = (k == 0 ? xr.x : k == 1 ? xr.y : k == 2 ? xr.z : xr.w) - xj[c];
+          r2 = fmaf(dl, dl, r2);
+#pragma unroll
+          for (int b = 0; b < P2; ++b) be[b] = fmaf(dl, wj[b][c], be[b]);
+#pragma unroll
+          for (int a = 0; a < P1; ++a) {
+            const float ui = k == 0 ? ur[a].x : k == 1 ? ur[a].y : k == 2 ? ur[a].z : ur[a].w;
+            al[a] = fmaf(dl, ui, al[a]);
+#pragma unroll
+            for (int b = 0; b < P2; ++b) ga[a][b] = fmaf(ui, wj[b][c], ga[a][b]);
+          }
+        }
+      }
+      // ---- coefficients (as in kdir_bwd_v4)
+      const float k = os * expf(-0.5f * r2 * il2);
+      float as[PA], bs[PB], das[PA], dbs[PB], hab[PA][PB];
+#pragma unroll
+      for (int a = 0; a < P1; ++a) as[a] = al[a] * il2;
+#pragma unroll
+      for (int b = 0; b < P2; ++b) bs[b] = be[b] * il2;
+      float qk = g[0][0];
+#pragma unroll
+      for (int b = 0; b < P2; ++b) {
+        dbs[b] = g[0][1 + b];
+        qk += dbs[b] * bs[b];
+      }
+#pragma unroll
+      for (int a = 0; a < P1; ++a) {
+        const float ga0 = g[1 + (a < P1 ? a : 0)][0];
+        das[a] = -ga0;
+        qk -= ga0 * as[a];
+#pragma unroll
+        for (int b = 0; b < P2; ++b) {
+          const float gab = g[1 + (a < P1 ? a : 0)][1 + b];
+          qk += gab * (ga[a][b] * il2 - as[a] * bs[b]);
+          das[a] -= gab * bs[b];
+          dbs[b] -= gab * as[a];
+          hab[a][b] = k * gab * il2;
+        }
+      }
+      const float e0 = -qk * k * il2;
+      float ea[PA], eb[PB];
+#pragma unroll
+      for (int a = 0; a < P1; ++a) ea[a] = k * das[a] * il2;
+#pragma unroll
+      for (int b = 0; b < P2; ++b) eb[b] = k * dbs[b] * il2;
+      // ---- accumulate over this row point
+#pragma unroll
+      for (int c4 = 0; c4 < DP; c4 += 4) {
+        const float4 xr = *reinterpret_cast<const float4*>(rb + c4);
+        float4 ur[PA];
+#pragma unroll
+        for (int a = 0; a < P1; ++a) ur[a] = *reinterpret_cast<const float4*>(rb + (1 + a) * DP + c4);
+#pragma unroll
+        for (int kk = 0; kk < 4; ++kk) {
+          const int c = c4 + kk;
+          const float dl = (kk == 0 ? xr.x : kk == 1 ? xr.y : kk == 2 ? xr.z : xr.w) - xj[c];
+          float tx = e0 * dl;
+#pragma unroll
+          for (int b = 0; b < P2; ++b) tx = fmaf(eb[b], wj[b][c], tx);
+          float tw[PB];
+#pragma unroll
+          for (int b = 0; b < P2; ++b) tw[b] = eb[b] * dl;
+#pragma unroll
+          for (int a = 0; a < P1; ++a) {
+            const float ui = kk == 0 ? ur[a].x : kk == 1 ? ur[a].y : kk == 2 ? ur[a].z : ur[a].w;
+            tx = fmaf(ea[a], ui, tx);
+#pragma unroll
+            for (int b = 0; b < P2; ++b) tw[b] = fmaf(hab[a][b], ui, tw[b]);
+          }
+          sx[c] -= tx;
+#pragma unroll
+          for (int b = 0; b < P2; ++b) sw[b][c] += tw[b];
+        }
+      }
+#pragma unroll
+      for (int a = 0; a < Q1; ++a)
+#pragma unroll
+        for (int b = 0; b < Q2; ++b) g[a][b] = gn[a][b];
+    }
+  }
+  if (!act) return;
+  double* prow = part + ((int64_t)blockIdx.y * n2 * Q2 + (int64_t)j * Q2) * d;   // rows (j, 0..P2) of kdir_bwd_reduce_rows
+#pragma unroll
+  for (int c = 0; c < DP; ++c)
+    if (c < d) {
+      prow[c] = (double)sx[c];
+#pragma unroll
+      for (int b = 0; b < P2; ++b) prow[(1 + b) * d + c] = (double)sw[b][c];
+    }
+}
+
 // ------------------------------------------------------------------------------------ backward (runtime p)
 // One thread per point pair, atomics into double accumulators.  Any p <= DSVGP_MAXP; not tuned.
 template <typename T, typename TK>
@@ -1233,11 +1413,11 @@ kdir_bwd_generic(const T* __restrict__ x1, const TK* __restrict__ u1, int n1, in
   }
 }
 
-// One warp per output row (i,a'): sums the column-chunk partials, applies the chain rule of the row
+// One warp per output row (i,a'): sums the column-chunk partials (TP: fp32 or fp64), applies the chain rule of the row
 // normalisation (RBFKernelDirectionalGrad.py:57) for direction rows, and ACCUMULATES scale*grad into the
 // double gradient buffers gx (n1,d) / gv (n1*p1,d).
-template <typename TK>
-__global__ void kdir_bwd_reduce_rows(const TK* __restrict__ part, int nchunk, int n1, int p1, int d,
+template <typename TP, typename TK>
+__global__ void kdir_bwd_reduce_rows(const TP* __restrict__ part, int nchunk, int n1, int p1, int d,
                                      const TK* __restrict__ u1, const TK* __restrict__ inv_norm, double scale,
                                      double* __restrict__ gx, double* __restrict__ gv) {
   const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
@@ -1446,7 +1626,7 @@ static int launch_bwd_blocked(const T* x1, const TK* u1, const TK* inv1, int n1,
   dim3 grid(nchunk, rt);
   kern<<<grid, 256, smem, st>>>(x1, u1, n1, x2, w2, n2, d, hyp, use_os, dK, lddk, dk_trans, chunk_pts, part, part_sc);
   CHECK_LAUNCH();
-  kdir_bwd_reduce_rows<TK><<<ceil_div(n1 * (P1 + 1), 8), 256, 0, st>>>(part, nchunk, n1, P1, d, u1, inv1, scale, gx, gv);
+  kdir_bwd_reduce_rows<TK, TK><<<ceil_div(n1 * (P1 + 1), 8), 256, 0, st>>>(part, nchunk, n1, P1, d, u1, inv1, scale, gx, gv);
   CHECK_LAUNCH();
   if (gsc) {
     kdir_bwd_reduce_scalars<<<1, 256, 0, st>>>(part_sc, rt * nchunk, gsc);
@@ -1495,7 +1675,7 @@ int kdir_bwd(const T* x1, const TK* u1, const TK* inv1, int n1, int p1, const T*
 #undef BV4V
       if (launched) {
         CHECK_LAUNCH();
-        kdir_bwd_reduce_rows<float><<<ceil_div(n1 * (p1 + 1), 8), 256, 0, st>>>(part, nt, n1, p1, d, u1, inv1, scale, gx, gv);
+        kdir_bwd_reduce_rows<float, float><<<ceil_div(n1 * (p1 + 1), 8), 256, 0, st>>>(part, nt, n1, p1, d, u1, inv1, scale, gx, gv);
         CHECK_LAUNCH();
         if (gsc) {
           kdir_bwd_reduce_scalars<<<1, 256, 0, st>>>(part_sc, nt * nrc, gsc);
@@ -1527,6 +1707,59 @@ int kdir_bwd(const T* x1, const TK* u1, const TK* inv1, int n1, int p1, const T*
   return DSVGP_OK;
 }
 
+// workspace (bytes) of kdir_bwd_cols: the fp64 chunk partials of the vectorised kernel, or what the blocked kernel needs for
+// the swapped problem (data side as the first argument, dK read transposed)
+template <typename TK>
+size_t kdir_bwd_cols_workspace(int n1, int p1, int n2, int p2, int d) {
+  const size_t blocked = kdir_bwd_workspace<TK>(n2, p2, n1, p1, d);
+  if (sizeof(TK) == 4 && bwd_v4_ok(n1, p1, n2, p2, d)) {
+    const size_t v4 = sizeof(double) * (size_t)cols_num_chunks(n1, n2) * n2 * (p2 + 1) * d + 256;
+    return v4 > blocked ? v4 : blocked;
+  }
+  return blocked;
+}
+
+// Accumulates scale * dL/dx2 into gx (n2,d) and scale * dL/dv2 into gv (n2*p2,d) (either may be null; double buffers) for
+// dL = sum(dK * K(x1, x2)).  Returns 1 when the vectorised fp32 kernel ran, 0 when the blocked kernel did (dk_trans = 1 on the
+// swapped problem: every shape and dtype, reading dK strided).
+template <typename T, typename TK>
+int kdir_bwd_cols(const T* x1, const TK* u1, int n1, int p1, const T* x2, const TK* w2, const TK* inv2, int n2, int p2, int d,
+                  const double* hyp, int use_os, const TK* dK, int64_t lddk, double scale, double* gx, double* gv, void* ws,
+                  size_t ws_bytes, cudaStream_t st) {
+  if (n1 <= 0 || n2 <= 0) return DSVGP_OK;
+  if (p1 < 0 || p2 < 0 || p1 > DSVGP_MAXP || p2 > DSVGP_MAXP || d <= 0) return DSVGP_ERR_ARG;
+  if (ws_bytes < kdir_bwd_cols_workspace<TK>(n1, p1, n2, p2, d)) return DSVGP_ERR_WORKSPACE;
+  if constexpr (sizeof(T) == 4 && sizeof(TK) == 4) {
+    if (bwd_v4_ok(n1, p1, n2, p2, d)) {
+      const int nchunk = cols_num_chunks(n1, n2), chunk_pts = ceil_div(n1, nchunk);
+      const int DPr = (d + 3) & ~3;
+      double* part = reinterpret_cast<double*>(ws);
+      dim3 grid(ceil_div(n2, COLS_TJ), nchunk);
+      int launched = 0;
+#define BCOL(A, B, DPV)                                                                                        \
+  if (!launched && p1 == A && p2 == B && DPr == DPV) {                                                         \
+    kdir_bwd_cols_v4<A, B, DPV><<<grid, COLS_TJ, 0, st>>>(x1, u1, n1, x2, w2, n2, d, hyp, use_os, dK, lddk,    \
+                                                         chunk_pts, part);                                     \
+    launched = 1;                                                                                              \
+  }
+#define BCOL_ALL(A, B) BCOL(A, B, 4) BCOL(A, B, 8) BCOL(A, B, 12) BCOL(A, B, 16)
+      BCOL_ALL(0, 0) BCOL_ALL(1, 1) BCOL_ALL(2, 2) BCOL_ALL(1, 0) BCOL_ALL(2, 0)
+      BCOL(0, 0, 20) BCOL(1, 1, 20) BCOL(2, 2, 20) BCOL(1, 0, 20) BCOL(2, 0, 20)
+#undef BCOL_ALL
+#undef BCOL
+      if (launched) {
+        CHECK_LAUNCH();
+        kdir_bwd_reduce_rows<double, float><<<ceil_div(n2 * (p2 + 1), 8), 256, 0, st>>>(part, nchunk, n2, p2, d, w2, inv2, scale,
+                                                                                         gx, gv);
+        CHECK_LAUNCH();
+        return 1;
+      }
+    }
+  }
+  return kdir_bwd<T, TK>(x2, w2, inv2, n2, p2, x1, u1, n1, p1, d, hyp, use_os, dK, lddk, 1, scale, gx, gv, nullptr, ws, ws_bytes,
+                         st);
+}
+
 // explicit instantiations: (T, TK) in {(f32,f32), (f64,f64), (f32,f64)}
 #define INST(T, TK)                                                                                             \
   template int normalize_dirs<T, TK>(const T*, int, int, TK*, TK*, cudaStream_t, int*, int*);                               \
@@ -1544,5 +1777,13 @@ template int kdir_diag<float>(int, int, const double*, int, float*, cudaStream_t
 template int kdir_diag<double>(int, int, const double*, int, double*, cudaStream_t);
 template size_t kdir_bwd_workspace<float>(int, int, int, int, int);
 template size_t kdir_bwd_workspace<double>(int, int, int, int, int);
+template size_t kdir_bwd_cols_workspace<float>(int, int, int, int, int);
+template size_t kdir_bwd_cols_workspace<double>(int, int, int, int, int);
+template int kdir_bwd_cols<float, float>(const float*, const float*, int, int, const float*, const float*, const float*, int, int,
+                                         int, const double*, int, const float*, int64_t, double, double*, double*, void*, size_t,
+                                         cudaStream_t);
+template int kdir_bwd_cols<double, double>(const double*, const double*, int, int, const double*, const double*, const double*,
+                                           int, int, int, const double*, int, const double*, int64_t, double, double*, double*,
+                                           void*, size_t, cudaStream_t);
 
 }  // namespace dsvgp

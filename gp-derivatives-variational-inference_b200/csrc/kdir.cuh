@@ -32,4 +32,13 @@ int kdir_bwd(const T* x1, const TK* u1, const TK* inv1, int n1, int p1, const T*
              int d, const double* hyp, int use_os, const TK* dK, int64_t lddk, int dk_trans, double scale,
              double* gx, double* gv, double* gsc, void* ws, size_t ws_bytes, cudaStream_t st);
 
+// data-side gradient (d/dx2, d/dv2) of the same product; returns 1 if the vectorised fp32 kernel ran, 0 for the blocked one
+template <typename TK>
+size_t kdir_bwd_cols_workspace(int n1, int p1, int n2, int p2, int d);
+
+template <typename T, typename TK>
+int kdir_bwd_cols(const T* x1, const TK* u1, int n1, int p1, const T* x2, const TK* w2, const TK* inv2, int n2, int p2, int d,
+                  const double* hyp, int use_os, const TK* dK, int64_t lddk, double scale, double* gx, double* gv, void* ws,
+                  size_t ws_bytes, cudaStream_t st);
+
 }  // namespace dsvgp

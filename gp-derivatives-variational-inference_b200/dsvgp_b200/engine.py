@@ -167,7 +167,8 @@ class Workspace:
         self.X = sq()
         self.Y, self.Psi, self.S = (e(Mq, Mq, dt=F64) for _ in range(3))
         self.gm = self.gLs = None      # allocated fresh by every backward pass (handed to autograd without a copy)
-        self.wx = None
+        self.gx = self.gVx = None      # (fp64) d/dx, d/dVx: allocated fresh by a backward pass that wants them
+        self.wx = self.invx = None     # normalised data-side directions and 1/|Vx|
         self.generation = 0
         self.canon = None          # (cidx, flag) of the data-side directions when detected canonical on device
 
@@ -353,14 +354,15 @@ class Engine:
     def _data_dirs(ws, Vx, T):
         """normalised data-side directions (+ on-device detection of canonical rows for the fp32 fast path)"""
         if not ws.p2:
-            ws.canon = None
+            ws.canon = ws.invx = None
             return None
         if T == F32:
-            wx, _, cidx, flag = ops.normalize_dirs_canon(Vx)
+            wx, ws.invx, cidx, flag = ops.normalize_dirs_canon(Vx)
             ws.canon = (cidx, flag)
             return wx
         ws.canon = None
-        return ops.normalize_dirs(Vx, T)[0]
+        wx, ws.invx = ops.normalize_dirs(Vx, T)
+        return wx
 
     @staticmethod
     def _w64(ws):
@@ -484,9 +486,31 @@ class Engine:
         ops.predict_finish(ws.pm, ws.pv, nq, ws.p2, f.hyp, ws.mu, ws.var, add_noise, PRED_JITTER)
 
     # ----------------------------------------------------------------------------------------------- backward
-    def _backward(self, ws, f, P, x, wx, gmu, gvar, add_noise, inv_num_data, reducer=None):
+    @staticmethod
+    def _input_grads(ws, f, P, x, wx, dKzx):
+        """d/dx and d/dVx (fp64, fresh) of the data side of K_zx from dK_zx.  They stay local to a minibatch shard: nothing here
+        enters the buffers that are summed over ranks."""
+        n, d = x.shape
+        ws.gx = torch.zeros(n, d, dtype=F64, device=x.device)
+        ws.gVx = torch.zeros(n * ws.p2, d, dtype=F64, device=x.device) if ws.p2 else None
+        ops.kdir_bwd_cols(P.Z, f.uzT, ws.p, x, wx, ws.invx, ws.p2, f.hyp, dKzx, ws.gx, ws.gVx)
+
+    @staticmethod
+    def _input_grad_dict(ws, x, Vx, gmu, names):
+        """{"x", "Vx", "y"} gradients in the model dtype (those in `names`): Vx gets exact zeros when the data side keeps no
+        derivative rows (p2 = 0: Vx influences nothing), y gets -d/dmu (the Gaussian data terms depend on y - mu only)."""
+        g = {}
+        if "x" in names:
+            g["x"] = ws.gx.to(x.dtype)
+        if "Vx" in names:
+            g["Vx"] = ws.gVx.to(x.dtype) if ws.gVx is not None else torch.zeros_like(Vx)
+        if "y" in names:
+            g["y"] = torch.neg(gmu)
+        return g
+
+    def _backward(self, ws, f, P, x, wx, gmu, gvar, add_noise, inv_num_data, reducer=None, want_inputs=False):
         """Gradients of a scalar whose derivatives w.r.t. (mean, variance) are (gmu, gvar), plus the KL gradient
-        scaled by -inv_num_data.  Results: ws.gm, ws.gLs (model dtype), ws.small (double).
+        scaled by -inv_num_data.  Results: ws.gm, ws.gLs (model dtype), ws.small (double); with want_inputs also ws.gx, ws.gVx.
 
         Order: the Gram product G = A diag(g_var) A^T comes FIRST, because [G | t] is what has to be summed over ranks:
         its all-reduce is started as soon as G exists (reducer.begin) and runs underneath dK_zx = L^-T dA and the K_zx
@@ -495,6 +519,7 @@ class Engine:
         T, Mq, nq = x.dtype, ws.Mq, ws.nq
         A, Ag, C, dKzx = ws.A, ws.B, ws.C, ws.Kzx
         ops.pred_bwd_scalars(gmu, gvar, ws.p2, f.hyp, add_noise, ws.sc[4:], ws.scratch)
+        ws.gx = ws.gVx = None
         tc = ws.tc and f.tc
         if ws.tch and f.tch:
             # 3xFP16: scales of dA and A_g from max|m|, max|g_mu|, max|g_var|, max|C| (order-independent maxima: deterministic)
@@ -533,6 +558,8 @@ class Engine:
                     if under_reduce:
                         ops.set_tc_persistent(True)
             ops.kdir_bwd(P.Z, f.uzT, f.invzT, ws.p, x, wx, ws.p2, f.hyp, dKzx, ws.gZ, ws.gVz, ws.sc[4:6])
+            if want_inputs:
+                self._input_grads(ws, f, P, x, wx, dKzx)
             # (E, E^T as fp32 + lo for the two M'^3 products of the tail were made by _assemble)
         else:
             ops.dA_apply(A, C, Ag, Mq, nq, P.m, gmu, gvar, ws.tp, ws.t,                  # C <- dA ; Ag ; t = A gmu
@@ -551,6 +578,8 @@ class Engine:
             else:
                 ops.gemm(self._wt(f), C, dKzx, ta=True, a_tri=TRI_UPPER, M=Mq, N=nq, K=Mq)
             ops.kdir_bwd(P.Z, f.uzT, f.invzT, ws.p, x, wx, ws.p2, f.hyp, dKzx, ws.gZ, ws.gVz, ws.sc[4:6])
+            if want_inputs:
+                self._input_grads(ws, f, P, x, wx, dKzx)
         if reducer is not None:
             reducer.end(ws.small)
         self._backward_tail(ws, f, P, T, inv_num_data, reducer)
@@ -661,7 +690,7 @@ class Engine:
 
     # ------------------------------------------------------------------------------------------ public: train
     def elbo_step(self, P, x, Vx, y, num_data, p, p2, through_likelihood=True, n_global=None, want_grads=True,
-                  objective="elbo", include_kl=True, reducer=None):
+                  objective="elbo", include_kl=True, reducer=None, input_grads=()):
         """One fused forward(+backward) of VariationalELBO(likelihood, model, num_data)(likelihood(model(x)), y)
         -- or, objective="pll", of PredictiveLogLikelihood (directional_vi.py:218-219).
 
@@ -671,7 +700,8 @@ class Engine:
         log_marginal's own application too (2 in the reference loop).  `variance` includes that many noises.
         include_kl=False leaves the KL term (value and gradient) to the caller: the shared-direction strategy's q(u) lives
         on M + p values, not on the M(p+1) inducing values the step sees.
-        reducer (distributed.Reducer or None): sums [G | t] and the small fp64 buffer over the ranks of a sharded step."""
+        reducer (distributed.Reducer or None): sums [G | t] and the small fp64 buffer over the ranks of a sharded step.
+        input_grads: names among "x", "Vx", "y" whose gradients the grads dict should also carry (this shard's own)."""
         self._validate(P, x, Vx, p, p2, y)
         T, dev = x.dtype, x.device
         n, d = x.shape
@@ -704,7 +734,7 @@ class Engine:
                     wx = self._data_dirs(ws, Vx, T)
                     # (allocated while the side stream is current, read by kernels of the caller's stream later in the step:
                     #  tell the caching allocator, so that a freed block is not handed out again before those have run)
-                    for t_ in (wx, *((f.uzT, f.invzT) if (f.p and T != F64) else ()), *(ws.canon or ())):
+                    for t_ in (wx, ws.invx, *((f.uzT, f.invzT) if (f.p and T != F64) else ()), *(ws.canon or ())):
                         if t_ is not None:
                             t_.record_stream(cur)
                     if f.tch:
@@ -732,15 +762,18 @@ class Engine:
                 ops.pll_terms(ws.mu, ws.var, y, 1.0 / nq_global, ws.gmu, ws.gvar, ws.sc, ws.scratch)
             else:
                 ops.elbo_terms(ws.mu, ws.var, y, f.hyp, 1.0 / nq_global, ws.gmu, ws.gvar, ws.sc, ws.scratch)
-            if want_grads:
+            want_inputs = "x" in input_grads or "Vx" in input_grads
+            if want_grads or want_inputs:
                 self._backward(ws, f, P, x, wx, ws.gmu, ws.gvar, through_likelihood, (1.0 / num_data) if include_kl else 0.0,
-                               reducer)
+                               reducer, want_inputs)
             elif reducer is not None:
                 reducer.end(ws.small)
             # everything the caller gets is enqueued BEFORE the one host synchronisation of the step (the Cholesky status
             # read), so the GPU never waits for the host at the end of a step
             elbo = ws.sc[0] - ws.kl[0] / num_data
-            grads = self._collect(ws, f, P, T, 1) if want_grads else None
+            grads = self._collect(ws, f, P, T, 1) if (want_grads or want_inputs) else None
+            if input_grads:
+                grads = {**(grads or {}), **self._input_grad_dict(ws, x, Vx, ws.gmu, input_grads)}
             mean, var = ws.mu.clone(), ws.var.clone()
             if capturing:
                 # CUDA-graph capture: no host synchronisation inside the captured region.  The factorisation status stays in
@@ -770,13 +803,17 @@ class Engine:
                 return (ws, f), ws.mu.clone(), ws.var.clone()
         raise NotPSDError("K_zz is not positive definite after adding jitter up to 1e-4 (psd_safe_cholesky ladder)")
 
-    def predictive_backward(self, ctx, P, x, gmu, gvar, add_noise):
+    def predictive_backward(self, ctx, P, x, gmu, gvar, add_noise, Vx=None, input_grads=()):
+        """input_grads: names among "x", "Vx" whose gradients the returned dict should also carry."""
         ws, f = ctx
         ws.small.zero_()
         min_var = 1e-10 if x.dtype == F64 else 1e-6
         gvar = torch.where(ws.var > min_var, gvar, torch.zeros_like(gvar)).contiguous()
-        self._backward(ws, f, P, x, ws.wx, gmu.contiguous(), gvar, add_noise, 0.0)
-        return self._collect(ws, f, P, x.dtype, 0)
+        self._backward(ws, f, P, x, ws.wx, gmu.contiguous(), gvar, add_noise, 0.0, want_inputs=bool(input_grads))
+        grads = self._collect(ws, f, P, x.dtype, 0)
+        if input_grads:
+            grads.update(self._input_grad_dict(ws, x, Vx, None, input_grads))
+        return grads
 
     # ------------------------------------------------------------------------------------------ public: eval
     @staticmethod
@@ -857,13 +894,15 @@ class Engine:
         predict_full (the reference's lazy predictive covariance is differentiable, DGVS.py:192-208)."""
         return self.predict_full(P, x, Vx, p, p2, add_noise, reuse_factor=False, return_ctx=True)
 
-    def full_backward(self, ctx, P, x, gmean, gcov, add_noise):
+    def full_backward(self, ctx, P, x, gmean, gcov, add_noise, Vx=None, input_grads=()):
         """Gradients of a scalar whose derivatives w.r.t. (mean, covariance) of q(f(X)) are (gmean, gcov).
         Sigma = K_xx + 1e-4 I + A^T D A (+ noise), D = S - I:  with Gs = gcov + gcov^T,
             dA = m gmean^T + D (A Gs),   G = 1/2 (A Gs) A^T  (then dA A^T = m t^T + 2 D G, t = A gmean, dL_s = tril(2 G L_s)),
         i.e. the same (dA, G, t) interface as the diagonal case, after which dK_zx = W^T dA, the assembly backward and the
         O(M'^3) tail are the training step's own (_backward_tail).  K_xx contributes to the lengthscale / outputscale only.
-        Evaluation sizes (BO candidates: n' of a few hundred to a few thousand): every product on the generic mma.sync GEMM."""
+        Evaluation sizes (BO candidates: n' of a few hundred to a few thousand): every product on the generic mma.sync GEMM.
+        input_grads: names among "x", "Vx" whose gradients the returned dict should also carry; x and Vx enter through K_zx
+        and through the dense K_xx (whose diagonal does not depend on them)."""
         ws, f = ctx
         T, Mq, nq = x.dtype, ws.Mq, ws.nq
         wx = ws.wx
@@ -884,13 +923,24 @@ class Engine:
         dKzx = ws.Kzx
         ops.gemm(self._wt(f), Bp, dKzx, ta=True, a_tri=TRI_UPPER, M=Mq, N=nq, K=Mq)             # dK_zx = L^-T dA
         ops.kdir_bwd(P.Z, f.uzT, f.invzT, ws.p, x, wx, ws.p2, f.hyp, dKzx, ws.gZ, ws.gVz, ws.sc[4:6])
-        # K_xx: only the kernel hyper-parameters depend on it (x and the data directions are inputs, not parameters).  Its DIAGONAL
-        # (closed form in ell, os) is already in pred_bwd_scalars' terms above: the assembly backward gets the off-diagonal part.
+        ws.gx = ws.gVx = None
+        if input_grads:
+            self._input_grads(ws, f, P, x, wx, dKzx)
+        # K_xx: of the parameters only the kernel hyper-parameters depend on it.  Its DIAGONAL (closed form in ell, os) is already in
+        # pred_bwd_scalars' terms above: the assembly backward gets the off-diagonal part.
         goff = gcov.clone()
         goff.diagonal().zero_()
         ops.kdir_bwd(x, wx if ws.p2 else None, None, ws.p2, x, wx if ws.p2 else None, ws.p2, f.hyp, goff, None, None, ws.sc[4:6])
+        if input_grads:
+            # x (and Vx) are both arguments of K_xx(x, x): the gradient w.r.t. the second equals the row-side gradient of the
+            # transposed upstream block, so the two sides are one row-side pass over goff + goff^T
+            gsym = goff + goff.transpose(0, 1)
+            ops.kdir_bwd(x, wx if ws.p2 else None, ws.invx, ws.p2, x, wx if ws.p2 else None, ws.p2, f.hyp, gsym, ws.gx, ws.gVx, None)
         self._backward_tail(ws, f, P, T, 0.0)
-        return self._collect(ws, f, P, T, 0)
+        grads = self._collect(ws, f, P, T, 0)
+        if input_grads:
+            grads.update(self._input_grad_dict(ws, x, Vx, None, input_grads))
+        return grads
 
     def sample_mvn(self, mean, cov, num_samples, generator=None):
         """num_samples draws of N(mean, cov): fp64 Cholesky of cov on the library's own blocked factorisation (same

@@ -426,19 +426,35 @@ class GaussianLikelihood(Module):
 _PARAM_ORDER = ("Z", "Vz", "m", "Ls_raw", "c", "raw_os", "raw_ell", "raw_noise")
 
 
+_INPUT_ORDER = ("x", "Vx", "y")
+
+
+def _inputs_wanted(needs):
+    """names of the inputs (x, Vx[, y]) whose entries of ctx.needs_input_grad are set, from position 1 on"""
+    return tuple(name for name, need in zip(_INPUT_ORDER, needs[1:]) if need)
+
+
+def _scaled_input_grads(grads, names, shapes, g_out):
+    """the input gradients of a backward pass scaled by the incoming gradient, shaped like the inputs (None where not wanted)"""
+    return [grads[name].reshape(shp) * g_out.to(grads[name].dtype) if name in names else None
+            for name, shp in zip(_INPUT_ORDER, shapes)]
+
+
 class _ElboStep(torch.autograd.Function):
-    """value = ELBO; the gradients w.r.t. every parameter are computed by the same fused GPU pass and handed
-    to autograd in backward (scaled by the incoming gradient)."""
+    """value = ELBO; the gradients w.r.t. every parameter -- and w.r.t. x, Vx, y when they require it -- are computed by the
+    same fused GPU pass and handed to autograd in backward (scaled by the incoming gradient)."""
 
     @staticmethod
     def forward(ctx, cfg, x, Vx, y, *params):
         P = types.SimpleNamespace(**dict(zip(_PARAM_ORDER, params)))
         want = any(ctx.needs_input_grad[4:])      # (grad mode is off inside forward; this is the reliable signal)
+        inputs = _inputs_wanted(ctx.needs_input_grad[:4])
         elbo, grads, mean, var = ENGINE.elbo_step(P, x, Vx, y, cfg["num_data"], cfg["p"], cfg["p2"],
                                                   cfg["through_likelihood"], cfg.get("n_global"), want_grads=want,
                                                   objective=cfg.get("objective", "elbo"), include_kl=cfg.get("include_kl", True),
-                                                  reducer=cfg.get("reducer"))
-        ctx.grads = grads
+                                                  reducer=cfg.get("reducer"), input_grads=inputs)
+        ctx.grads, ctx.inputs = grads, inputs
+        ctx.input_shapes = tuple(None if t is None else t.shape for t in (x, Vx, y))
         ctx.mark_non_differentiable(mean, var)
         return elbo.to(x.dtype), mean, var
 
@@ -454,7 +470,8 @@ class _ElboStep(torch.autograd.Function):
             scaled = torch._foreach_mul([g for _, g in wanted], g_elbo.to(wanted[0][1].dtype))
             for (k, _), g in zip(wanted, scaled):
                 out[k] = g
-        return (None, None, None, None, *out)
+        ins = _scaled_input_grads(grads, ctx.inputs, ctx.input_shapes, g_elbo) if ctx.inputs else [None] * 3
+        return (None, *ins, *out)
 
 
 class _Predictive(torch.autograd.Function):
@@ -465,7 +482,7 @@ class _Predictive(torch.autograd.Function):
     def forward(ctx, cfg, x, Vx, *params):
         P = types.SimpleNamespace(**dict(zip(_PARAM_ORDER, params)))
         ectx, mean, var = ENGINE.predictive_forward(P, x, Vx, cfg["p"], cfg["p2"], cfg["add_noise"])
-        ctx.ectx, ctx.P, ctx.x, ctx.cfg = ectx, P, x, cfg
+        ctx.ectx, ctx.P, ctx.x, ctx.Vx, ctx.cfg = ectx, P, x, Vx, cfg
         ctx.generation = (ectx[0].generation, ectx[1].generation)     # bumped by EVERY later user of the workspace / factor
         return mean, var
 
@@ -474,12 +491,15 @@ class _Predictive(torch.autograd.Function):
         if (ctx.ectx[0].generation, ctx.ectx[1].generation) != ctx.generation:
             raise RuntimeError("dsvgp_b200: the predictive workspace was overwritten by a later forward pass before "
                                "backward ran; call backward before evaluating the model again on the same shape")
-        grads = ENGINE.predictive_backward(ctx.ectx, ctx.P, ctx.x, gmu, gvar, ctx.cfg["add_noise"])
+        inputs = _inputs_wanted(ctx.needs_input_grad[:3])
+        grads = ENGINE.predictive_backward(ctx.ectx, ctx.P, ctx.x, gmu, gvar, ctx.cfg["add_noise"], Vx=ctx.Vx,
+                                           input_grads=inputs)
         out = []
         for name, need in zip(_PARAM_ORDER, ctx.needs_input_grad[3:]):
             g = grads.get(name)
             out.append(g if (need and g is not None) else None)
-        return (None, None, None, *out)
+        ins = [grads[name] if name in inputs else None for name in _INPUT_ORDER[:2]]
+        return (None, *ins, *out)
 
 
 class _FullPredictive(torch.autograd.Function):
@@ -491,7 +511,7 @@ class _FullPredictive(torch.autograd.Function):
     def forward(ctx, cfg, x, Vx, *params):
         P = types.SimpleNamespace(**dict(zip(_PARAM_ORDER, params)))
         ectx, mean, cov = ENGINE.full_forward(P, x, Vx, cfg["p"], cfg["p2"], cfg["add_noise"])
-        ctx.ectx, ctx.P, ctx.x, ctx.cfg = ectx, P, x, cfg
+        ctx.ectx, ctx.P, ctx.x, ctx.Vx, ctx.cfg = ectx, P, x, Vx, cfg
         ctx.generation = (ectx[0].generation, ectx[1].generation)
         return mean, cov
 
@@ -500,12 +520,14 @@ class _FullPredictive(torch.autograd.Function):
         if (ctx.ectx[0].generation, ctx.ectx[1].generation) != ctx.generation:
             raise RuntimeError("dsvgp_b200: the predictive workspace was overwritten by a later forward pass before "
                                "backward ran; call backward before evaluating the model again on the same shape")
-        grads = ENGINE.full_backward(ctx.ectx, ctx.P, ctx.x, gmean, gcov, ctx.cfg["add_noise"])
+        inputs = _inputs_wanted(ctx.needs_input_grad[:3])
+        grads = ENGINE.full_backward(ctx.ectx, ctx.P, ctx.x, gmean, gcov, ctx.cfg["add_noise"], Vx=ctx.Vx, input_grads=inputs)
         out = []
         for name, need in zip(_PARAM_ORDER, ctx.needs_input_grad[3:]):
             g = grads.get(name)
             out.append(g if (need and g is not None) else None)
-        return (None, None, None, *out)
+        ins = [grads[name] if name in inputs else None for name in _INPUT_ORDER[:2]]
+        return (None, *ins, *out)
 
 
 class PredictiveDistribution:
@@ -530,12 +552,16 @@ class PredictiveDistribution:
     def _params(self):
         return self._strategy._param_list(self._likelihood)
 
+    def _differentiable(self, params):
+        """autograd path: gradients are enabled and a parameter or an input (x, derivative_directions) requires them"""
+        return torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in (self._x, self._Vx, *params))
+
     def _evaluate(self):
         if self._cache is None:
             st = self._strategy
             cfg = dict(p=st._p(), p2=st._p2(), add_noise=self._noise_mult)
             params = self._params()
-            if torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in params):
+            if self._differentiable(params):
                 self._cache = _Predictive.apply(cfg, self._x, self._Vx, *params)
             else:
                 P = types.SimpleNamespace(**dict(zip(_PARAM_ORDER, params)))
@@ -568,7 +594,7 @@ class PredictiveDistribution:
         if self._full is None:
             st = self._strategy
             params = self._params()
-            if torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in params):
+            if self._differentiable(params):
                 cfg = dict(p=st._p(), p2=st._p2(), add_noise=self._noise_mult)
                 self._full = _FullPredictive.apply(cfg, self._x, self._Vx, *params)
             else:

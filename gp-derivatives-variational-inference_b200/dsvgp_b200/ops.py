@@ -101,6 +101,19 @@ def kdir_bwd(x1, u1, inv1, p1, x2, w2, p2, hyp, dK, gx, gv, gsc, use_os=True, dk
          gv if p1 else None, gsc, ws, ws.numel())
 
 
+def kdir_bwd_cols(x1, u1, p1, x2, w2, inv2, p2, hyp, dK, gx, gv, use_os=True, scale=1.0):
+    """Accumulate scale*dL/dx2 into gx and scale*dL/dv2 into gv (float64): the data-side gradient of K(x1, x2) given dK
+    (laid out as kdir_fwd writes K).  True when the dedicated fp32 kernel ran, False when the blocked one read dK transposed."""
+    n1, d = x1.shape
+    n2 = x2.shape[0]
+    nbytes = call_raw("dsvgp_kdir_bwd_cols_workspace_" + suffix(dK.dtype), n1, p1, n2, p2, d)
+    ws = _workspace(nbytes, x1.device, "kdir_bwd_cols")
+    rc = call("dsvgp_kdir_bwd_cols_" + suffix(dK.dtype), x1, u1 if p1 else None, n1, p1, x2, w2 if p2 else None,
+              inv2 if (p2 and gv is not None) else None, n2, p2, d, hyp, int(use_os), dK, _ld(dK), float(scale), gx,
+              gv if p2 else None, ws, ws.numel())
+    return rc == 1
+
+
 def gemm(A, B, C, ta=False, tb=False, alpha=1.0, beta=0.0, a_tri=TRI_NONE, b_tri=TRI_NONE, c_tri=0, D=None,
          M=None, N=None, K=None, C2=None, D2=None):
     """C[:M,:N] = alpha*op(A)[:M,:K] @ op(B)[:K,:N] + beta*(D or C); optionally also C2 = C + D2.

@@ -99,6 +99,19 @@ int dsvgp_kdir_bwd_f32(const float* x1, const float* u1, const float* inv1, int 
 int dsvgp_kdir_bwd_f64(const double* x1, const double* u1, const double* inv1, int n1, int p1, const double* x2, const double* w2, int n2, int p2, int d, const double* hyp, int use_os, const double* dK, int64_t lddk, int dk_trans, double scale, double* gx, double* gv, double* gsc, void* ws, size_t ws_bytes, dsvgp_stream_t s);
 int dsvgp_kdir_bwd_f32f64(const float* x1, const double* u1, const double* inv1, int n1, int p1, const float* x2, const double* w2, int n2, int p2, int d, const double* hyp, int use_os, const double* dK, int64_t lddk, int dk_trans, double scale, double* gx, double* gv, double* gsc, void* ws, size_t ws_bytes, dsvgp_stream_t s);
 
+/* Data-side ("column") gradient of dsvgp_kdir_fwd_*: the gradient w.r.t. the SECOND argument (the data points x2 and their
+ * directions v2 of K_zx), given dK laid out as the forward writes K (n1(p1+1) x n2(p2+1), row-major).  ACCUMULATES
+ *   gx (n2,d)      += scale * dL/dx2         (NULL to skip)
+ *   gv (n2*p2,d)   += scale * dL/dv2 (chain rule through the normalisation included, inv2 = 1/|v2|; NULL to skip)
+ * in double.  fp32 with d <= 20, n2 >= 512 and (p1, p2) in {(0,0), (1,1), (2,2), (1,0), (2,0)} runs a dedicated kernel that
+ * reads dK once, row by row and coalesced, recomputes K and sums fp64 partials in a fixed order (no atomics), and returns 1;
+ * every other shape and fp64 run dsvgp_kdir_bwd_* with dk_trans = 1 on the swapped problem (dK read strided) and return 0.
+ * Results agree to rounding.  No length- or outputscale gradient (dsvgp_kdir_bwd_* gives those). */
+size_t dsvgp_kdir_bwd_cols_workspace_f32(int n1, int p1, int n2, int p2, int d);
+size_t dsvgp_kdir_bwd_cols_workspace_f64(int n1, int p1, int n2, int p2, int d);
+int dsvgp_kdir_bwd_cols_f32(const float* x1, const float* u1, int n1, int p1, const float* x2, const float* w2, const float* inv2, int n2, int p2, int d, const double* hyp, int use_os, const float* dK, int64_t lddk, double scale, double* gx, double* gv, void* ws, size_t ws_bytes, dsvgp_stream_t s);
+int dsvgp_kdir_bwd_cols_f64(const double* x1, const double* u1, int n1, int p1, const double* x2, const double* w2, const double* inv2, int n2, int p2, int d, const double* hyp, int use_os, const double* dK, int64_t lddk, double scale, double* gx, double* gv, void* ws, size_t ws_bytes, dsvgp_stream_t s);
+
 /* Cholesky of the jittered K_zz and the inverse factor -- _cholesky_factor / psd_safe_cholesky
  * (DirectionalGradVariationalStrategy.py:72-75) and TriangularLazyTensor.inv_matmul (:181,:183).
  * dsvgp_chol_plan: padded size Mp = nb0 << nlev for an Mq x Mq matrix.  dsvgp_pad_identity_f64 writes the identity
