@@ -96,6 +96,10 @@ int dsvgp_pad_identity_f64(double* A, int64_t ld, int Mq, int Mp, dsvgp_stream_t
 int dsvgp_chol_f64(double* Awork, int64_t lda, double* L, int64_t ldl, double* W, int64_t ldw, int Mp, int nb0, int nlev, int* info, dsvgp_stream_t s) {
   return chol_factor_inverse(Awork, lda, L, ldl, W, ldw, Mp, nb0, nlev, info, ST(s));
 }
+size_t dsvgp_chol_bwd_workspace_f64(int n) { return chol_bwd_workspace(n); }
+int dsvgp_chol_bwd_f64(const double* L, int64_t ldl, const double* W, int64_t ldw, const double* Lbar, int64_t ldlb, double* Abar, int64_t lda, int n, void* ws, size_t ws_bytes, dsvgp_stream_t s) {
+  return chol_backward(L, ldl, W, ldw, Lbar, ldlb, Abar, lda, n, ws, ws_bytes, ST(s));
+}
 
 int dsvgp_set_potrf_debug(void* p) { set_potrf_debug(static_cast<long long*>(p)); return 0; }
 int dsvgp_collect_grads_f32(const double* small, int nZ, int nV, const double* hyp, int noise_mode, float* out, dsvgp_stream_t s) { return collect_grads<float>(small, nZ, nV, hyp, noise_mode, out, ST(s)); }

@@ -24,6 +24,7 @@
 #include "chol.cuh"
 #include "common.cuh"
 #include "gemm.cuh"
+#include "misc.cuh"
 
 namespace dsvgp {
 
@@ -1326,6 +1327,47 @@ int chol_factor_inverse(double* Awork, int64_t lda, double* L, int64_t ldl, doub
     return DSVGP_ERR_LAUNCH;
   }
   return DSVGP_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// Cholesky backward of a general SPD matrix A = L L^T (what autograd of torch.linalg.cholesky gives):
+//     dA = 1/2 (S + S^T),   S = W^T Phi(L^T dL) W,   W = L^-1,   Phi = lower triangle with the diagonal halved.
+// Three triangular fp64 products and two elementwise passes on the caller's stream; P and Y live in the workspace.
+static int64_t chol_bwd_ld(int n) { return ((int64_t)n + 1) & ~(int64_t)1; }   // even: 16-byte rows for the epilogue stores
+
+size_t chol_bwd_workspace(int n) { return n < 1 ? 0 : (size_t)(2 * (int64_t)n * chol_bwd_ld(n)) * sizeof(double); }
+
+static bool ranges_overlap(const void* a, size_t na, const void* b, size_t nb) {
+  const uintptr_t x = reinterpret_cast<uintptr_t>(a), y = reinterpret_cast<uintptr_t>(b);
+  return x < y + nb && y < x + na;
+}
+
+int chol_backward(const double* L, int64_t ldl, const double* W, int64_t ldw, const double* Lbar, int64_t ldlb, double* dA,
+                  int64_t lda, int n, void* ws, size_t ws_bytes, cudaStream_t st) {
+  if (!L || !W || !Lbar || !dA || !ws || n < 1 || ldl < n || ldw < n || ldlb < n || lda < n) return DSVGP_ERR_ARG;
+  // the fp64 products load their operands one element per 8-byte cp.async: every base must be 8-byte aligned
+  if (((reinterpret_cast<uintptr_t>(L) | reinterpret_cast<uintptr_t>(W) | reinterpret_cast<uintptr_t>(Lbar) |
+        reinterpret_cast<uintptr_t>(dA) | reinterpret_cast<uintptr_t>(ws)) & 7) != 0)
+    return DSVGP_ERR_ARG;
+  const size_t need = chol_bwd_workspace(n);
+  if (ws_bytes < need) return DSVGP_ERR_WORKSPACE;
+  auto span = [n](int64_t ld) { return (size_t)(((int64_t)(n - 1) * ld + n) * (int64_t)sizeof(double)); };
+  const void* in[3] = {L, W, Lbar};
+  const size_t in_span[3] = {span(ldl), span(ldw), span(ldlb)};
+  for (int i = 0; i < 3; ++i)
+    if (ranges_overlap(dA, span(lda), in[i], in_span[i]) || ranges_overlap(ws, need, in[i], in_span[i])) return DSVGP_ERR_ARG;
+  if (ranges_overlap(ws, need, dA, span(lda))) return DSVGP_ERR_ARG;
+
+  const int64_t ldp = chol_bwd_ld(n);
+  double* P = static_cast<double*>(ws);
+  double* Y = P + (int64_t)n * ldp;
+  int rc;
+  // P = tril(L^T dL): only the lower triangle of dL is loaded; tiles above the diagonal of P are not computed
+  if ((rc = gemm1<double>(true, false, n, n, n, 1.0, L, ldl, Lbar, ldlb, 0.0, P, ldp, TRI_UPPER, TRI_LOWER, 1, st))) return rc;
+  if ((rc = phi_lower(P, ldp, Y, ldp, n, st))) return rc;                                     // Y = Phi(P), reads tril(P)
+  if ((rc = gemm1<double>(false, false, n, n, n, 1.0, Y, ldp, W, ldw, 0.0, P, ldp, TRI_LOWER, TRI_LOWER, 1, st))) return rc;   // P = Phi W (lower)
+  if ((rc = gemm1<double>(true, false, n, n, n, 1.0, W, ldw, P, ldp, 0.0, dA, lda, TRI_UPPER, TRI_LOWER, 0, st))) return rc;   // S = W^T P
+  return symmetrize(dA, lda, n, st);
 }
 
 }  // namespace dsvgp

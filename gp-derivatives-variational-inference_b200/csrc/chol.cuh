@@ -13,6 +13,11 @@ void chol_plan(int Mq, int* Mp, int* nb0, int* nlev);
 int chol_factor_inverse(double* Awork, int64_t lda, double* L, int64_t ldl, double* W, int64_t ldw, int Mp, int nb0,
                         int nlev, int* info, cudaStream_t st);
 
+// dA = sym(W^T Phi(L^T dL) W) from the lower triangles of L, W = L^-1 and dL (contract: include/dsvgp_b200.h)
+size_t chol_bwd_workspace(int n);
+int chol_backward(const double* L, int64_t ldl, const double* W, int64_t ldw, const double* Lbar, int64_t ldlb, double* dA,
+                  int64_t lda, int n, void* ws, size_t ws_bytes, cudaStream_t st);
+
 // 1: round-1 diagonal-block kernel (in-kernel DMMA prologue, scalar updates); 2 (default): diag_prepare + all-DMMA block kernel
 void set_chol_variant(int v);
 int get_chol_variant();

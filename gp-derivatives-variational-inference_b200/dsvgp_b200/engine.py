@@ -942,9 +942,11 @@ class Engine:
             grads.update(self._input_grad_dict(ws, x, Vx, None, input_grads))
         return grads
 
-    def sample_mvn(self, mean, cov, num_samples, generator=None):
+    def sample_mvn(self, mean, cov, num_samples, generator=None, base=None, keep=False):
         """num_samples draws of N(mean, cov): fp64 Cholesky of cov on the library's own blocked factorisation (same
-        jitter ladder as psd_safe_cholesky), then mean + z L^T as one triangular product."""
+        jitter ladder as psd_safe_cholesky), then mean + z L^T as one triangular product.  base: fp64 (num_samples, n')
+        standard normals used as z instead of fresh ones.  keep: also return (L, W, z, jitter) for sample_backward, with
+        L, W = L^-1 the padded Mp x Mp factors (the identity padding decouples their leading n' x n' block)."""
         nq = mean.shape[0]
         dev = mean.device
         Mp, nb0, nlev = ops.chol_plan(nq)
@@ -961,10 +963,29 @@ class Engine:
                 break
         else:
             raise NotPSDError("the predictive covariance is not positive definite after adding jitter up to 1e-4")
-        z = torch.randn(num_samples, nq, dtype=F64, device=dev, generator=generator)
+        z = torch.randn(num_samples, nq, dtype=F64, device=dev, generator=generator) if base is None else base
         out = torch.empty(num_samples, nq, dtype=F64, device=dev)
         ops.gemm(z, L, out, tb=True, b_tri=TRI_UPPER, M=num_samples, N=nq, K=nq)      # z L^T
-        return (out + mean.to(F64)).to(mean.dtype)
+        res = (out + mean.to(F64)).to(mean.dtype)
+        return (res, (L, W, z, extra)) if keep else res
+
+    def sample_backward(self, L, W, z, gout, want_base=False):
+        """Gradients of draws = mean + z L^T (sample_mvn with keep=True) given gout = dloss/d draws (num, n'):
+        (d mean, d cov, d z or None).  d L = tril(gout^T z) and d cov = sym(W^T Phi(L^T dL) W) (ops.chol_backward); the
+        jitter of the factorisation is a constant, so d cov is the gradient w.r.t. the covariance the caller passed."""
+        num, nq = z.shape
+        dev = z.device
+        gout = gout.to(F64).contiguous()
+        gmean = gout.sum(0)
+        Lbar = torch.empty(nq, _round_up(nq, 2), dtype=F64, device=dev)[:, :nq]
+        ops.gemm(gout, z, Lbar, ta=True, c_tri=1, M=nq, N=nq, K=num)               # lower triangle of gout^T z
+        gcov = torch.empty(nq, _round_up(nq, 2), dtype=F64, device=dev)[:, :nq]
+        ops.chol_backward(L[:nq, :nq], W[:nq, :nq], Lbar, gcov, nq)
+        gz = None
+        if want_base:
+            gz = torch.empty(num, nq, dtype=F64, device=dev)
+            ops.gemm(gout, L, gz, b_tri=TRI_LOWER, M=num, N=nq, K=nq)                # gout L
+        return gmean, gcov, gz
 
     def invalidate(self):
         for f in self._fac.values():

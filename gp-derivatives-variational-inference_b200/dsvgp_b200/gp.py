@@ -530,11 +530,33 @@ class _FullPredictive(torch.autograd.Function):
         return (None, *ins, *out)
 
 
+class _MVNSample(torch.autograd.Function):
+    """Reparameterised draws mean + L z, L = chol(cov + jitter I) and z the given base samples (fp64 (num, n')) or fresh
+    standard normals: gpytorch's MultivariateNormal.rsample.  backward gives (d mean, d cov, d base) through the fp64
+    Cholesky backward; autograd carries (d mean, d cov) on into _FullPredictive.  L, W = L^-1 and z are fresh tensors
+    held here, so a later draw cannot overwrite them."""
+
+    @staticmethod
+    def forward(ctx, mean, cov, base, num):
+        z = None if base is None else base.detach().to(device=mean.device, dtype=torch.float64).contiguous()
+        out, (L, W, z, _) = ENGINE.sample_mvn(mean, cov, num, base=z, keep=True)
+        ctx.L, ctx.W, ctx.z = L, W, z
+        ctx.base_meta = None if base is None else (base.device, base.dtype)
+        return out
+
+    @staticmethod
+    def backward(ctx, gout):
+        need_mean, need_cov, need_base = ctx.needs_input_grad[:3]
+        gmean, gcov, gz = ENGINE.sample_backward(ctx.L, ctx.W, ctx.z, gout, want_base=need_base)
+        return (gmean.to(gout.dtype) if need_mean else None, gcov.to(gout.dtype) if need_cov else None,
+                gz.to(*ctx.base_meta) if need_base else None, None)
+
+
 class PredictiveDistribution:
     """Lazy q(f(X)) returned by a variational strategy (stands in for gpytorch's MultivariateNormal with a lazy
     covariance).  Only what the reference's callers consume is offered: .mean / .loc, .variance, .stddev
-    (directional_vi.py:256-257, :297-298), plus the full predictive covariance (.covariance_matrix, differentiable) and
-    .sample / .rsample (SURVEY.md section 8f rank 4; the draw itself is not reparameterised)."""
+    (directional_vi.py:256-257, :297-298), plus the full predictive covariance (.covariance_matrix) and the reparameterised
+    draws .rsample / .sample (SURVEY.md section 8f rank 4), all differentiable."""
 
     def __init__(self, strategy, x, Vx, likelihood=None, noise_mult=0):
         self._strategy, self._x, self._Vx, self._likelihood = strategy, x, Vx, likelihood
@@ -612,17 +634,35 @@ class PredictiveDistribution:
     lazy_covariance_matrix = covariance_matrix
 
     def rsample(self, sample_shape=torch.Size(), base_samples=None):
-        mean, cov = (t.detach() for t in self._evaluate_full())      # (the draw is not reparameterised: no gradient through it)
-        shape = torch.Size(sample_shape)
+        """Reparameterised draws mean + L z of shape sample_shape + event_shape, as gpytorch's MultivariateNormal.rsample:
+        differentiable w.r.t. everything the mean and covariance depend on (parameters, x, derivative_directions) and w.r.t.
+        base_samples.  base_samples (..., n'): the standard normals z, used in fp64; sample_shape is then its leading
+        dimensions.  L is always the exact fp64 Cholesky factor of the covariance, with psd_safe_cholesky's jitter ladder
+        (gpytorch 1.4 switches to a Lanczos root above max_cholesky_size; this library does not)."""
+        nq = self.event_shape[0]
+        if base_samples is not None:
+            if base_samples.shape[-1:] != self.event_shape:
+                raise RuntimeError(f"the size of base_samples (minus sample shape dimensions) should agree with the size of "
+                                   f"self.loc: expected ...{tuple(self.event_shape)} but got {tuple(base_samples.shape)}")
+            shape = base_samples.shape[:-1]
+            base = base_samples.reshape(-1, nq)
+        else:
+            shape = torch.Size(sample_shape)
+            base = None
         num = int(math.prod(shape)) if len(shape) else 1
-        out = ENGINE.sample_mvn(mean, cov, num)
-        return out.reshape(*shape, mean.shape[0])
+        mean, cov = self._evaluate_full()
+        if torch.is_grad_enabled() and (mean.requires_grad or cov.requires_grad or (base is not None and base.requires_grad)):
+            out = _MVNSample.apply(mean, cov, base, num)
+        else:
+            z = None if base is None else base.detach().to(device=mean.device, dtype=torch.float64).contiguous()
+            out = ENGINE.sample_mvn(mean.detach(), cov.detach(), num, base=z)
+        return out.reshape(*shape, nq)
 
     def sample(self, sample_shape=torch.Size(), base_samples=None):
         """preds.sample(torch.Size([n_samples])) -> (n_samples, n') as gpytorch's MultivariateNormal.sample
         (experiments/rover/test_turbo.py:138)."""
         with torch.no_grad():
-            return self.rsample(sample_shape)
+            return self.rsample(sample_shape, base_samples)
 
 
 # ------------------------------------------------------------------------------------------------ objectives

@@ -297,6 +297,15 @@ def cholesky_inverse(Awork, L, W, nb0, nlev, info):
     call("dsvgp_chol_f64", Awork, _ld(Awork), L, _ld(L), W, _ld(W), Awork.shape[0], nb0, nlev, info)
 
 
+def chol_backward(L, W, Lbar, out, n=None):
+    """out[:n,:n] = sym(W^T Phi(L^T Lbar) W): the gradient w.r.t. A = L L^T given Lbar = dloss/dL (fp64; the lower
+    triangles of L, W = L^-1 and Lbar are read)."""
+    n = L.shape[0] if n is None else n
+    ws = _workspace(call_raw("dsvgp_chol_bwd_workspace_f64", int(n)), L.device, "chol_bwd")
+    call("dsvgp_chol_bwd_f64", L, _ld(L), W, _ld(W), Lbar, _ld(Lbar), out, _ld(out), int(n), ws, ws.numel())
+    return out
+
+
 def cast2d(src, dst, rows=None, cols=None, tril=False):
     rows = src.shape[0] if rows is None else rows
     cols = src.shape[1] if cols is None else cols

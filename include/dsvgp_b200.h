@@ -167,6 +167,19 @@ int dsvgp_set_chol_lookahead(int on);
 int dsvgp_set_potrf_debug(void* buf);
 int dsvgp_chol_f64(double* Awork, int64_t lda, double* L, int64_t ldl, double* W, int64_t ldw, int Mp, int nb0, int nlev, int* info, dsvgp_stream_t s);
 
+/* Cholesky backward of a general SPD matrix (what autograd of torch.linalg.cholesky gives; the gradient of the draws
+ * mean + L z of a predictive distribution w.r.t. its covariance): from L (lower, as dsvgp_chol_f64 writes it), W = L^-1 (lower)
+ * and Lbar = dloss/dL, writes the full symmetric n x n
+ *     Abar = 1/2 (S + S^T),   S = W^T Phi(L^T Lbar) W,   Phi = lower triangle with the diagonal halved.
+ * Only the lower triangles of L, W and Lbar are read.  Three triangular fp64 products and two elementwise passes, all on `s`;
+ * P = tril(L^T Lbar) and Phi(P) W go to the workspace (dsvgp_chol_bwd_workspace_f64(n) bytes).  The products load their
+ * operands one double per 8-byte cp.async, so every pointer (L, W, Lbar, Abar, ws) must be 8-byte aligned; leading dimensions
+ * need only be >= n.  DSVGP_ERR_ARG, with nothing enqueued, for a NULL pointer, n < 1, a leading dimension < n, a misaligned
+ * pointer, or Abar or the workspace overlapping the address range of an input (or each other); DSVGP_ERR_WORKSPACE for a
+ * workspace that is too small.  Abar's columns past n and the workspace past its size are not touched. */
+size_t dsvgp_chol_bwd_workspace_f64(int n);
+int dsvgp_chol_bwd_f64(const double* L, int64_t ldl, const double* W, int64_t ldw, const double* Lbar, int64_t ldlb, double* Abar, int64_t lda, int n, void* ws, size_t ws_bytes, dsvgp_stream_t s);
+
 /* C = alpha*op(A)*op(B) + beta*C, triangle-aware, batched -- every dense product of the strategy
  * (DirectionalGradVariationalStrategy.py:181-205) and of its backward.  fp32 uses 3xTF32 (fp32-accurate).
  * D != NULL: C = alpha*op(A)*op(B) + beta*D (D not batched); D == NULL: the addend is C itself.
