@@ -530,7 +530,8 @@ int gemm(bool ta, bool tb, int M, int N, int K, T alpha, const T* A, int64_t lda
          T* C, int64_t ldc, int a_tri, int b_tri, int c_tri, int batch, int64_t sA, int64_t sB, int64_t sC,
          cudaStream_t st, const T* D, int64_t ldd, T* C2, int64_t ldc2, const T* D2, int64_t ldd2, int c_off) {
   if (M <= 0 || N <= 0 || batch <= 0) return DSVGP_OK;
-  if (!A || !B || !C || K < 0 || (C2 && !D2)) return DSVGP_ERR_ARG;
+  // K = 0 reads neither operand (C = beta * D): an empty operand, whose pointer torch reports as NULL, is accepted there
+  if (!C || K < 0 || (K > 0 && (!A || !B)) || (C2 && !D2)) return DSVGP_ERR_ARG;
   GemmParams<T> p{A, B, C, D, C2, D2, M, N, K, lda, ldb, ldc, ldd, ldc2, ldd2, sA, sB, sC, alpha, beta, a_tri, b_tri, c_tri, c_off};
   dim3 grid(ceil_div(N, BN), ceil_div(M, BM), batch);
   if constexpr (sizeof(T) == 8) {

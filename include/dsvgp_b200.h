@@ -183,7 +183,9 @@ int dsvgp_chol_bwd_f64(const double* L, int64_t ldl, const double* W, int64_t ld
 /* C = alpha*op(A)*op(B) + beta*C, triangle-aware, batched -- every dense product of the strategy
  * (DirectionalGradVariationalStrategy.py:181-205) and of its backward.  fp32 uses 3xTF32 (fp32-accurate).
  * D != NULL: C = alpha*op(A)*op(B) + beta*D (D not batched); D == NULL: the addend is C itself.
- * C2 != NULL: a second output C2 = C + D2 is written by the same epilogue (used for B' = E^T A, B = A + B'). */
+ * C2 != NULL: a second output C2 = C + D2 is written by the same epilogue (used for B' = E^T A, B = A + B').
+ * K = 0 gives C = beta*D (or beta*C) and reads neither operand, so A and B may then be NULL.  M = 0, N = 0 or batch = 0
+ * return DSVGP_OK with nothing written; K < 0, C2 without D2, and a NULL C (or A, B with K > 0) are DSVGP_ERR_ARG. */
 int dsvgp_gemm_f32(int ta, int tb, int M, int N, int K, double alpha, const float* A, int64_t lda, const float* B, int64_t ldb, double beta, float* C, int64_t ldc, int a_tri, int b_tri, int c_tri, int batch, int64_t sA, int64_t sB, int64_t sC, const float* D, int64_t ldd, float* C2, int64_t ldc2, const float* D2, int64_t ldd2, dsvgp_stream_t s);
 int dsvgp_gemm_f64(int ta, int tb, int M, int N, int K, double alpha, const double* A, int64_t lda, const double* B, int64_t ldb, double beta, double* C, int64_t ldc, int a_tri, int b_tri, int c_tri, int batch, int64_t sA, int64_t sB, int64_t sC, const double* D, int64_t ldd, double* C2, int64_t ldc2, const double* D2, int64_t ldd2, dsvgp_stream_t s);
 
